@@ -54,7 +54,43 @@ def parse_args():
                     help="url_like = BASELINE configs[1] (the bench line the driver records); int_filter = configs[2]; "
                          "shipdate = configs[3] (TPC-H SF100 l_shipdate range, one GPU's shard of the 8-way split per rank); "
                          "clickbench_sweep = configs[4] (scan stage of the 43 ClickBench queries, bench_sweep.py)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="url_like: after the timed steps, write the filtered URLs the last step returned as DIR/url_*.npy, so that "
+                         "two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "url_like" or args.impl != "ours"):
+        ap.error("--dump-outputs is written by --workload url_like --impl ours")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_strings(out_dir: str, name: str, arr):
+    """The Utf8 array `arr` as <name>_offsets.npy (float64, from 0) and <name>_bytes.npy (float32, the UTF-8 bytes), both exact,
+    with <name>_rows.npy (float64) the positions of the rows written: all of them, or when that would take more than
+    DUMP_BYTES, a sample of rows fixed by seed 0 and the row lengths, in row order."""
+    import numpy as np
+    import pyarrow as pa
+
+    def offsets(a):
+        return np.frombuffer(a.buffers()[1], dtype=np.int32)[a.offset:a.offset + len(a) + 1].astype(np.int64)
+
+    lens = np.diff(offsets(arr))
+    order = np.random.default_rng(0).permutation(len(arr))
+    # 8 + 8 + 4 * len bytes per row; the last offset and the three .npy headers fit in 1 KB
+    fits = int(np.searchsorted(np.cumsum(16 + 4 * lens[order]), DUMP_BYTES - 1024, side="right"))
+    rows = np.arange(len(arr)) if fits == len(arr) else np.sort(order[:fits])
+    if fits < len(arr):
+        arr = arr.take(pa.array(rows))
+    offs = offsets(arr)
+    data = np.frombuffer(arr.buffers()[2] or b"", dtype=np.uint8)[offs[0]:offs[-1]]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, f"{name}_offsets.npy"), (offs - offs[0]).astype(np.float64))
+    np.save(os.path.join(out_dir, f"{name}_bytes.npy"), data.astype(np.float32))
 
 
 def recorded_traffic(rows: int, entries: int):
@@ -731,13 +767,14 @@ def main():
 
         bench_sweep.main(args, rank, world, local_rank)
         return
-    run_url_like(args, rank, world, local_rank)
+    run_url_like(args, rank, world, local_rank, dump_dir=args.dump_outputs)
 
 
-def run_url_like(args, rank, world, local_rank, emit=True, source=None, rows=None, secondary=True):
-    """BASELINE configs[1] — the driver's bench line. `source`: "synthetic" (synth/lc_synth.c: the 100 M-row column the
+def run_url_like(args, rank, world, local_rank, emit=True, source=None, rows=None, secondary=True, dump_dir=None):
+    """BASELINE configs[1] — the headline bench line. `source`: "synthetic" (synth/lc_synth.c: the 100 M-row column the
     metric is quoted on) or "sample" (URLs resampled from the reference's 24 586-row ClickBench sample, synth/hits.py: the
-    real column's dictionary sizes, lengths and compressibility; reported beside it under config.secondary)."""
+    real column's dictionary sizes, lengths and compressibility; reported beside it under config.secondary). `dump_dir`:
+    rank 0 writes there the filtered URLs of every rank that the last timed step gathered (dump_strings)."""
     source = source or args.url_source
     import numpy as np
     import pyarrow as pa
@@ -904,6 +941,8 @@ def run_url_like(args, rank, world, local_rank, emit=True, source=None, rows=Non
     grows_in_timed = gather.grows - grows_before
     # what the e2e arm below is compared with: THIS rank's own filtered batch, downloaded from the gathered slots
     local_last = gather.to_arrow([rank])
+    if dump_dir and rank == 0:
+        dump_strings(dump_dir, "url", gather.to_arrow())
 
     # where a step's time goes (untimed, after the measurement): device events between the three calls of a step
     ph = [[], [], [], []]

@@ -8,6 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 import pyarrow as pa
@@ -16,19 +17,19 @@ _HERE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "c")
 _LIB = None
 
 
-def build(force: bool = False) -> None:
-    """gcc -O3 -march=native: always rebuilt on the machine that will time it."""
-    args = ["make", "-C", _HERE] + (["-B"] if force else [])
-    subprocess.run(args, check=True, stdout=subprocess.DEVNULL)
+def _load_fresh_build() -> C.CDLL:
+    """gcc -O3 -march=native on the machine that will time it, into a temporary directory: the tree may be read-only."""
+    with tempfile.TemporaryDirectory() as d:
+        so = os.path.join(d, "liblc_oracle.so")
+        subprocess.run(["make", "-C", _HERE, "-B", f"OUT={so}"], check=True, stdout=subprocess.DEVNULL)
+        return C.CDLL(so)
 
 
 def lib(rebuild: bool = False) -> C.CDLL:
     global _LIB
     if _LIB is None:
         so = os.path.join(_HERE, "liblc_oracle.so")
-        if rebuild or not os.path.exists(so):
-            build(force=True)
-        l = C.CDLL(so)
+        l = _load_fresh_build() if rebuild or not os.path.exists(so) else C.CDLL(so)
         vp, u32, u64, i64 = C.c_void_p, C.c_uint32, C.c_uint64, C.c_int64
         l.lco_int_encode.restype = vp
         l.lco_int_encode.argtypes = [vp, vp, u32, C.c_int, C.c_int]

@@ -1,7 +1,7 @@
 """ClickBench `hits`-shaped batches for the 43-query sweep (BASELINE.json configs[4], SURVEY.md §8d row 5).
 
 Rows are drawn with replacement from the 24 586-row sample of the real table that ships with the reference
-(synth/hits_sample.parquet, made by synth/make_sample.py), in runs: a batch keeps the sample's locality by taking
+(tests/golden/hits_sample.parquet, made by synth/make_sample.py), in runs: a batch keeps the sample's locality by taking
 consecutive sample rows from a random start, so per-batch dictionary sizes and bit widths look like the real column's
 (URL ~0.23 distinct values per row, EventTime a narrow window, flag columns one or two values). Two things the sample
 lacks are added: the token `google` is spliced into URL with probability 4e-5, as configs[1] does (paper Table 1: Q20
@@ -25,7 +25,7 @@ JULY_1_2013 = 15887  # days since 1970-01-01; the sample's only EventDate is 159
 
 class HitsSample:
     def __init__(self):
-        self.table = pq.read_table(os.path.join(_HERE, "hits_sample.parquet"))
+        self.table = pq.read_table(os.path.join(os.path.dirname(_HERE), "tests", "golden", "hits_sample.parquet"))
         self.n = self.table.num_rows
         self.cols = {c: self.table[c].combine_chunks() for c in self.table.column_names}
 
